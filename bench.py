@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native reflect-sampling-nerf hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload train|render] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload train|render] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -20,6 +20,8 @@ N > 1) with HOST (pinned) ray / pixel buffers, H2D + D2H copies inside the timed
 on the GPU inside the step, the e2e path receives them from the host: the two differ by one small kernel vs 655 KB of H2D.)
 `--impl reference` times the oracle restatement of the reference's PyTorch path on the host CPU cores
 (the reference itself cannot be imported: nerfstudio is absent, SURVEY.md §8c).
+`--dump-outputs DIR` writes what the timed path computed in its last timed step as DIR/<name>.npy (rank 0; see
+step_outputs_to_host): the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -108,6 +110,45 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": self.samples[0][1] if self.samples else None,
                 "reasons": reasons, "samples": len(self.samples), "power_w": pw[len(pw) // 2] if pw else None,
                 "power_limit_w": getattr(self, "power_limit_w", None), "power_note": "NVML board power, ~1 s average", "source": "nvml", "error": self.err}
+
+
+DUMP_RAYS, DUMP_SAMPLE_RAYS, DUMP_MAX_BYTES = 16384, 1024, 64 << 20
+
+
+def step_outputs_to_host(outputs, loss=None, field=None):
+    """What a caller of the timed path holds after its last step, copied to the host as float32 / float64 numpy arrays:
+    the per-ray outputs of get_outputs, and for a training step the loss and the updated field parameters.  Per-ray
+    outputs are those of a fixed, seeded sample of DUMP_RAYS rays (all of them for a batch no larger); per-sample outputs
+    ([rays, samples, c]) those of the first DUMP_SAMPLE_RAYS rays of the sample.  `rays` = the sampled ray indices."""
+    import numpy as np
+
+    def host(t):
+        t = t.detach().cpu()
+        return t.numpy().astype(np.float64 if t.dtype in (torch.float64, torch.int64, torch.int32) else np.float32)
+
+    n = next(iter(outputs.values())).shape[0]
+    rays = torch.arange(n)
+    if n > DUMP_RAYS:
+        rays = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_RAYS].sort().values
+    arrays = {"rays": rays.double().numpy()}
+    for k, v in outputs.items():
+        rows = rays[:DUMP_SAMPLE_RAYS] if v.dim() == 3 else rays
+        arrays[k] = host(v[rows.to(v.device)])
+    if loss is not None:
+        arrays["loss"] = host(loss)
+    if field is not None:
+        arrays.update({"param." + k: host(p) for k, p in field.named_parameters()})
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs exceed {DUMP_MAX_BYTES}")
+    return arrays
+
+
+def dump_step_outputs(arrays, out_dir: str) -> None:
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------ oracle arms
@@ -252,7 +293,7 @@ def run_b200(args):
                 ev.record()
                 loss_ring["ev"][slot] = ev
                 loss_ring["i"] += 1
-            return None
+            return loss
         out = model(bundle)
         if e2e:
             return out["mid_rgb_fine"].cpu(), out["mid_reflect_fine"].cpu()
@@ -306,12 +347,12 @@ def run_b200(args):
         if mode in ("eager", "graph") and world > 1:
             model.field.__dict__["_allreduce_events"] = []
         counters["launches"] = 0
-        evs = []
+        evs, last = [], None
         for _ in range(steps):
             flush.zero_()                       # L2 flush between timed iterations (outside the event pairs)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            run()
+            last = run()
             e1.record()
             evs.append((e0, e1))
             if mode != "e2e":
@@ -323,6 +364,7 @@ def run_b200(args):
         per_step = [a.elapsed_time(b) for a, b in evs]
         ms = sum(per_step)
         timed.last_per_step = per_step
+        timed.last_result = graph_state["loss"] if mode == "graph" else last     # the loss (train) / outputs (render)
         t = torch.tensor([ms], device=dev, dtype=torch.float64)
         mine = t.clone()
         if world > 1:
@@ -354,6 +396,11 @@ def run_b200(args):
     if sampler:
         sampler.stop_flag.set()
         sampler.join(timeout=2)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results, before the eager and e2e passes below train the model further
+        dumped = (step_outputs_to_host(stepper.last_outputs, timed.last_result, model.field) if train
+                  else step_outputs_to_host(timed.last_result))
     n_masked = [int(m) for m in masked] if masked else []
     # the same K steps eagerly, every instrumented kernel bracketed by CUDA events on the launching stream: the roofline's
     # launch durations (and the launch count of one step)
@@ -472,6 +519,8 @@ def run_b200(args):
             line["vs_cuda_baseline"] = {"fp32": value / cuda_base["fp32"], "fp16_autocast": value / cuda_base["fp16_autocast"]}
         sys.stdout.flush()
         os.write(json_fd, (json.dumps(line) + "\n").encode())
+    if dumped is not None:
+        dump_step_outputs(dumped, args.dump_outputs)
     if world > 1:
         dist.destroy_process_group()
 
@@ -493,6 +542,10 @@ def main():
                     help="CUDA-graph the training step (auto: single GPU only)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cuda-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float32 / float64, "
+                         "at most 64 MB): per-ray outputs, and for training the loss and the updated field parameters; "
+                         "with several GPUs, rank 0's rays only")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     args.scaling = "weak"
@@ -501,6 +554,8 @@ def main():
         total = 640000 if args.config == "C3" else 65536
         args.rays = (total + world - 1) // world
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs dumps the b200 path (--impl b200)")
         run_reference(args)
     else:
         run_b200(args)

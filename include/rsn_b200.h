@@ -181,12 +181,15 @@ int rsn_field_backward(const void* wblob_t, const void* x_stash, int mode, const
 int64_t rsn_field_dy_stash_bytes(int64_t n_points);
 
 /* ---- K5 backward, wgrad -----------------------------------------------------------------------------
- * dW = dY^T X and db = sum dY of every Linear of the field over all points of a pass, ACCUMULATED (fp32
- * atomics) into grad_blob, whose regions rsn_field_wgrad_layout describes (HOST pointers: offsets[2j] = dW
- * offset, offsets[2j+1] = db offset or -1, shapes[2j], shapes[2j+1] = rows, cols; returns the job count).
+ * dW = dY^T X and db = sum dY of every Linear of the field over all points of a pass, ACCUMULATED into grad_blob,
+ * whose regions rsn_field_wgrad_layout describes (HOST pointers: offsets[2j] = dW offset, offsets[2j+1] = db offset
+ * or -1, shapes[2j], shapes[2j+1] = rows, cols; returns the job count).  workspace (rsn_field_wgrad_workspace_bytes,
+ * 16-byte aligned, no initial contents) holds the per-CTA partial sums, added into grad_blob in a fixed order: the
+ * same inputs give the same gradient every run.  One workspace per launch in flight.
  * n_rays_dev != NULL: the pass covers min(*n_rays_dev * points_per_ray, n_points) points. */
-int rsn_field_wgrad(const void* x_stash, const void* dy_stash, int64_t n_points, float* grad_blob,
+int rsn_field_wgrad(const void* x_stash, const void* dy_stash, int64_t n_points, float* grad_blob, void* workspace,
                     const int* n_rays_dev, int64_t points_per_ray, rsn_stream_t stream);
+int64_t rsn_field_wgrad_workspace_bytes(void);
 int rsn_field_wgrad_layout(int64_t* host_offsets, int64_t* host_shapes, int64_t* total_floats);
 
 /* Completes the gradient blob once per step, after the last rsn_field_wgrad (and after the all-reduce): the bottleneck

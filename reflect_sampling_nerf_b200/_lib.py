@@ -42,7 +42,8 @@ _SIGNATURES = {
     "rsn_field_blob_t_bytes": ([], c_int64),
     "rsn_field_backward": ([P, P, I32, P, P, P, P, I64, I64, P, P, P, P, P, P, P, P], c_int),
     "rsn_field_dy_stash_bytes": ([I64], c_int64),
-    "rsn_field_wgrad": ([P, P, I64, P, P, I64, P], c_int),
+    "rsn_field_wgrad": ([P, P, I64, P, P, P, I64, P], c_int),
+    "rsn_field_wgrad_workspace_bytes": ([], c_int64),
     "rsn_field_wgrad_layout": ([P, P, P], c_int),
     "rsn_field_wgrad_finish": ([P, P, P, P, P], c_int),
     "rsn_unpack_grads": ([P, P, P], c_int),

@@ -12,8 +12,10 @@
 // for the chunk-major blocks, SWIZZLE_128B ones for the encodings) they are directly the A = dY^T and B = X operands of
 //   D[out, in] (+)= sum over 16 points  dY[pt, out] * X[pt, in]            (tcgen05.mma, fp32 in TMEM)
 // One CTA owns one job = (layer, all <=256 output features, <=256 input features) and a contiguous range of
-// tiles (split-K over points); its accumulators stay in TMEM for the whole range and are flushed once with
-// fp32 atomics.  db comes from the same shared-memory dY slabs, summed by the otherwise idle epilogue warps.
+// tiles (split-K over points); its accumulators stay in TMEM for the whole range and are stored once into the CTA's
+// slot of the caller's workspace; wgrad_reduce_kernel then adds the slots of every job into the blob in split order, so
+// the gradient is the same from run to run.  db comes from the same shared-memory dY slabs, summed by the otherwise idle
+// epilogue warps.
 //
 // HBM-bound: algorithmic bytes = (loaded dY blocks + n_blocks) * 16 KB per tile and job; 82 block reads = 1.31 MB per tile
 // over the 12 active jobs (10.25 KB per point) against 2 * 618k * 128 = 158 MFLOP per tile.
@@ -109,15 +111,31 @@ extern "C" int rsn_field_wgrad_finish(float* grad_blob, const float* w_bott, con
   return 0;
 }
 
+namespace {
+constexpr int MAX_WGRAD_CTAS = 160;   // one wave on a B200 (148 SMs); bounds the workspace
+}
+
+extern "C" int64_t rsn_field_wgrad_workspace_bytes(void) {
+  int64_t part_len = 0;
+  for (int j = 0; j < kNumJobs; ++j) {
+    const int64_t m = kJobs[j].m_blocks * 64;
+    part_len = std::max(part_len, m * kJobs[j].n_blocks * 64 + (kJobs[j].has_db ? m : 0));
+  }
+  return (int64_t)MAX_WGRAD_CTAS * part_len * (int64_t)sizeof(float);
+}
+
 extern "C" int rsn_field_wgrad(const void* x_stash, const void* dy_stash, int64_t n_points, float* grad_blob,
-                               const int* n_rays_dev, int64_t points_per_ray, cudaStream_t stream) {
+                               void* workspace, const int* n_rays_dev, int64_t points_per_ray, cudaStream_t stream) {
   RSN_ARG(n_points >= 0, "rsn_field_wgrad: bad shape");
   RSN_ARG(!n_rays_dev || (points_per_ray >= 1 && points_per_ray < (1 << 20)), "rsn_field_wgrad: bad points_per_ray");
   if (n_points == 0) return 0;
-  RSN_ARG(x_stash && dy_stash && grad_blob, "rsn_field_wgrad: null pointer");
+  RSN_ARG(x_stash && dy_stash && grad_blob && workspace, "rsn_field_wgrad: null pointer");
+  RSN_ARG(((uintptr_t)grad_blob & 15) == 0 && ((uintptr_t)workspace & 15) == 0,
+          "rsn_field_wgrad: grad_blob and workspace must be 16-byte aligned");
   RSN_ARG(((uintptr_t)x_stash & 15) == 0 && ((uintptr_t)dy_stash & 15) == 0, "rsn_field_wgrad: stashes must be 16-byte aligned");
   WParams p;
-  const int cta = fill_wgrad_params(p, x_stash, dy_stash, n_points, grad_blob, rsn_num_sms());
+  const int cta = fill_wgrad_params(p, x_stash, dy_stash, n_points, grad_blob, std::min(rsn_num_sms(), MAX_WGRAD_CTAS));
+  p.part = (float*)workspace;
   p.n_rays_dev = n_rays_dev;
   p.pts_per_ray = n_rays_dev ? (int)points_per_ray : 1;
   const size_t smem = (size_t)RING_BYTES + 1024;
@@ -125,6 +143,8 @@ extern "C" int rsn_field_wgrad(const void* x_stash, const void* dy_stash, int64_
   RSN_CUDA(rsn_ensure_smem(field_wgrad_kernel, (int)smem, done));
   field_wgrad_kernel<<<cta, W_THREADS, smem, stream>>>(p);
   RSN_LAUNCH_CHECK("field_wgrad_kernel");
+  wgrad_reduce_kernel<<<dim3(32, kNumJobs), 256, 0, stream>>>(p);
+  RSN_LAUNCH_CHECK("wgrad_reduce_kernel");
   if (p.debug & 16) {
     static unsigned long long t[2][160];
     RSN_CUDA(cudaStreamSynchronize(stream));

@@ -28,6 +28,7 @@ struct WJob {
   int a_cm, b_cm;        // 1: the dY / X blocks are chunk-major images (field_layout.cuh), 0: swizzled images
   int out_off, db_off;   // float offsets into the gradient blob: dW [64 m_blocks][64 n_blocks], db or -1
   int cta_begin, n_ctas;
+  int part_off, part_len;  // this job's partial sums in the workspace: split k at part_off + k * part_len floats (dW, then db)
 };
 struct WParams {
   const uint8_t* x;      // forward stash  [n_tiles][STASH_BLOCKS][16 KB]
@@ -36,6 +37,7 @@ struct WParams {
   const int* n_rays_dev; // optional device-side ray count (bounce passes): tiles = ceil(min(*n_rays_dev, rays) * pts_per_ray / 128)
   int pts_per_ray;
   float* grad;
+  float* part;           // workspace: every CTA's partial dW / db, added into grad in split order by wgrad_reduce_kernel
   int n_jobs;
   int debug;   // RSN_WGRAD_DEBUG (test build only): 1 = MMA only (no loads, no db), 2 = loads only (no MMA)
   WJob jobs[MAX_JOBS];
@@ -224,8 +226,9 @@ __device__ __forceinline__ void wgrad_body(const WParams& p) {
             const float t = warp_sum(acc[c][i]);
             if (lane == ((c * 8 + i) & 31)) mine[(c * 8 + i) >> 5] = t;
           }
-        atomicAdd(p.grad + job.db_off + blk * 64 + lane, mine[0]);
-        atomicAdd(p.grad + job.db_off + blk * 64 + 32 + lane, mine[1]);
+        float* db = p.part + job.part_off + (size_t)split * job.part_len + m_out * 64 * nb * 64 + blk * 64;
+        db[lane] = mine[0];
+        db[32 + lane] = mine[1];
       }
       mbar_wait(&bars.acc_full, 0);
       tc_fence_after();
@@ -233,16 +236,15 @@ __device__ __forceinline__ void wgrad_body(const WParams& p) {
       const int row = q * 32 + lane;
       const int N = nb * 64;
       for (int h = 0; h < ((p.debug & 4) ? 0 : m_out / 2); ++h) {
-        float* out = p.grad + job.out_off + (size_t)(h * 128 + row) * N;
+        float* out = p.part + job.part_off + (size_t)split * job.part_len + (size_t)(h * 128 + row) * N;
         for (int c0 = 0; c0 < N; c0 += 32) {
           uint32_t v[32];
           tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + h * 256 + c0, v);
           tmem_ld_wait();
 #pragma unroll
-          for (int i = 0; i < 32; i += 4)   // 16-byte vector reductions: 4x fewer L2 atomic transactions
-            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(out + c0 + i), "f"(__uint_as_float(v[i])),
-                         "f"(__uint_as_float(v[i + 1])), "f"(__uint_as_float(v[i + 2])), "f"(__uint_as_float(v[i + 3]))
-                         : "memory");
+          for (int i = 0; i < 32; i += 4)
+            *reinterpret_cast<float4*>(out + c0 + i) = make_float4(__uint_as_float(v[i]), __uint_as_float(v[i + 1]),
+                                                                   __uint_as_float(v[i + 2]), __uint_as_float(v[i + 3]));
         }
       }
     }
@@ -259,6 +261,36 @@ __device__ __forceinline__ void wgrad_body(const WParams& p) {
 
 __global__ void __launch_bounds__(W_THREADS, 1) field_wgrad_kernel(const __grid_constant__ WParams p) {
   wgrad_body(p);
+}
+
+// Adds the partial sums of every job's CTAs into the gradient blob, in split order: the same fp32 sums every run.
+// grid (blocks, jobs); a CTA that had no tile wrote nothing and is skipped; db rows past the loaded dY blocks are not
+// written by the wgrad (the blob keeps its value there, as it did with atomics).
+__global__ void __launch_bounds__(256) wgrad_reduce_kernel(const __grid_constant__ WParams p) {
+  const WJob job = p.jobs[blockIdx.y];
+  if (job.n_ctas == 0 || (p.debug & 4)) return;
+  int n_tiles = p.n_tiles;
+  if (p.n_rays_dev) {
+    const int64_t pts = (int64_t)max(__ldg(p.n_rays_dev), 0) * p.pts_per_ray;
+    n_tiles = (int)min((int64_t)n_tiles, (pts + TILE - 1) / TILE);
+  }
+  const bool interleave = !(p.debug & 8);
+  const int dw = job.m_blocks * 64 * job.n_blocks * 64;
+  const int db_rows = (job.db_off >= 0 && (p.debug & 3) != 1) ? job.a_load * 64 : 0;
+  for (int e = (blockIdx.x * blockDim.x + threadIdx.x) * 4; e < dw + db_rows; e += gridDim.x * blockDim.x * 4) {
+    float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int k = 0; k < job.n_ctas; ++k) {
+      const int t0 = interleave ? k : (int)(((int64_t)n_tiles * k) / job.n_ctas);
+      const int t1 = interleave ? n_tiles : (int)(((int64_t)n_tiles * (k + 1)) / job.n_ctas);
+      if (t1 <= t0) continue;
+      const float4 v = *reinterpret_cast<const float4*>(p.part + job.part_off + (size_t)k * job.part_len + e);
+      s.x += v.x, s.y += v.y, s.z += v.z, s.w += v.w;
+    }
+    float4* g = reinterpret_cast<float4*>(p.grad + job.out_off + e);     // db follows dW in the blob, as in the workspace
+    float4 o = *g;
+    o.x += s.x, o.y += s.y, o.z += s.z, o.w += s.w;
+    *g = o;
+  }
 }
 
 // The 12 jobs of one pass.  Gradient blob regions (fp32): dW [64 m_blocks][64 n_blocks] row-major, then db.
@@ -327,7 +359,7 @@ inline int fill_wgrad_params(WParams& p, const void* x_stash, const void* dy_sta
     ++n_of[best];
     ++used;
   }
-  int64_t off = 0;
+  int64_t off = 0, part = 0;
   int cta = 0;
   for (int j = 0; j < kNumJobs; ++j) {
     WJob& w = p.jobs[j];
@@ -342,6 +374,9 @@ inline int fill_wgrad_params(WParams& p, const void* x_stash, const void* dy_sta
     w.db_off = kJobs[j].has_db ? (int)off : -1;
     if (kJobs[j].has_db) off += w.m_blocks * 64;
     w.cta_begin = cta, w.n_ctas = n_of[j];
+    w.part_len = w.m_blocks * 64 * w.n_blocks * 64 + (kJobs[j].has_db ? w.m_blocks * 64 : 0);
+    w.part_off = (int)part;
+    part += (int64_t)n_of[j] * w.part_len;
     cta += n_of[j];
   }
   return cta;

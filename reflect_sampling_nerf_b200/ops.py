@@ -489,10 +489,12 @@ def field_backward(wblob_t: Tensor, stash: Tensor, mode: int, origins, dirs, are
 
 def field_wgrad(stash: Tensor, dy_stash: Tensor, n_points: int, grad_blob: Tensor, count: Optional[Tensor] = None,
                 points_per_ray: int = 1) -> None:
-    """K5 wgrad: accumulates dW / db of every Linear over the pass into grad_blob (fp32, wgrad_layout())."""
+    """K5 wgrad: accumulates dW / db of every Linear over the pass into grad_blob (fp32, wgrad_layout()), in a fixed
+    order (the same gradient every run).  The partial-sum workspace comes from the caching allocator, per call."""
+    ws = torch.empty(_lib.lib().rsn_field_wgrad_workspace_bytes(), dtype=torch.uint8, device=grad_blob.device)
     with _Prof("field_wgrad_kernel", n_points, count, n_points // max(points_per_ray, 1)):
-        _lib.call("rsn_field_wgrad", _lib.ptr(stash), _lib.ptr(dy_stash), n_points, _lib.ptr(grad_blob), _cnt(count),
-                  points_per_ray, _lib.stream())
+        _lib.call("rsn_field_wgrad", _lib.ptr(stash), _lib.ptr(dy_stash), n_points, _lib.ptr(grad_blob), _lib.ptr(ws),
+                  _cnt(count), points_per_ray, _lib.stream())
 
 
 def wgrad_finish(grad_blob: Tensor, w_bott: Tensor, b_bott: Tensor, w_mid: Tensor) -> None:

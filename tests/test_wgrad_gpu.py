@@ -59,6 +59,27 @@ def test_wgrad_matches_matmul(n_tiles):
             assert offs[2 * j + 1] == -1
 
 
+def test_wgrad_sums_are_the_same_from_launch_to_launch():
+    """The CTAs of a job add their split-K sums into the blob in split order: repeated launches on the same stashes give
+    bit-identical gradients (accumulated on top of a non-zero blob, as the passes of one backward do)."""
+    g = torch.Generator().manual_seed(5)
+    n_tiles = 160
+    xs = torch.randint(0, 256, (n_tiles, STASH_BLOCKS * 16384 + 36864), generator=g, dtype=torch.uint8)
+    xs = (xs & 0x3f).cuda()            # small finite bf16 values (high bytes < 0x40)
+    dys = (torch.randint(0, 256, (n_tiles, DY_BLOCKS, 16384), generator=g, dtype=torch.uint8) & 0x3d).cuda()
+    total = ops.wgrad_layout()[2]
+    start = torch.randn(total, generator=g).cuda()
+    blobs = []
+    for _ in range(4):
+        blob = start.clone()
+        ops.field_wgrad(xs, dys, n_tiles * 128, blob)
+        blobs.append(blob)
+    torch.cuda.synchronize()
+    assert torch.isfinite(blobs[0]).all() and not torch.equal(blobs[0], start)
+    for b in blobs[1:]:
+        assert torch.equal(b, blobs[0])
+
+
 def test_wgrad_finish_derives_the_bottleneck_gradients():
     """rsn_field_wgrad_finish on a random blob against the algebra it implements (and its host mirror in ops)."""
     g = torch.Generator().manual_seed(3)
